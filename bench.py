@@ -19,6 +19,11 @@ scene (default 1, exactly configs[1]).
 
 Multi-GPU: replicas only (the rasterizer has no trainable parameters, so there is no gradient
 all-reduce on this path); ranks render disjoint scenes, time is the max over ranks.
+
+--dump-outputs DIR writes what the last timed step returned (rank 0) as DIR/<name>.npy, float32, so
+that two builds run with the same arguments (hence the same seeded inputs) can be compared output for
+output: `image` [1, V, 3, H, W] whole, and `grad_<input>` for each Gaussian input, at a fixed seeded
+sample of Gaussians (dump_rows) that keeps the files under 64 MB.
 """
 from __future__ import annotations
 
@@ -33,6 +38,7 @@ import threading
 import time
 from pathlib import Path
 
+import numpy as np
 import torch
 
 ROOT = Path(__file__).resolve().parent
@@ -160,6 +166,25 @@ def render_step(d, d_img, views, state_out=None):
                        IMAGE, bg, *leaves, state_out=state_out)
     grads = torch.autograd.grad(img, leaves, d_img)
     return img, grads
+
+
+DUMP_GAUSSIANS = 65536          # gradient rows written by --dump-outputs (1/6 of configs[1]'s Gaussians)
+DUMP_LIMIT = 64 * 10**6         # bytes
+
+
+def dump_rows(P: int) -> torch.Tensor:
+    """The Gaussians whose gradients --dump-outputs writes: a fixed seeded sample, in ascending order."""
+    g = torch.Generator().manual_seed(0)
+    return torch.randperm(P, generator=g)[:DUMP_GAUSSIANS].sort().values
+
+
+def step_outputs(img, grads, rows) -> dict:
+    """Host float32 copies of what one step returns to its caller: the image whole, and the gradient of each
+    Gaussian input at `rows` (axis 1 is the Gaussian axis of every input)."""
+    out = {"image": img.detach()}
+    for k, gr in zip(GAUSS_KEYS, grads):
+        out["grad_" + k] = gr.index_select(1, rows.to(gr.device))
+    return {k: v.float().cpu().numpy() for k, v in out.items()}
 
 
 def capture_step(d, d_img, views):
@@ -310,8 +335,8 @@ def main():
     isolate_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=400)
-    ap.add_argument("--warmup", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 400; 2 with --impl reference)")
+    ap.add_argument("--warmup", type=int, default=None, help="warm-up steps (default 10; 1 with --impl reference)")
     ap.add_argument("--impl", default="native", choices=["native", "reference"])
     ap.add_argument("--views", type=int, default=1, help="target views per step (one scene)")
     ap.add_argument("--pool", type=int, default=4, help="distinct scenes cycled (> L2 in total)")
@@ -322,15 +347,24 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="issue every step from Python instead of replaying a CUDA graph")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's outputs to DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    reference = args.impl == "reference"
+    if args.steps is None:
+        args.steps = 2 if reference else 400
+    if args.warmup is None:
+        args.warmup = 1 if reference else 10
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and reference:
+        ap.error("--dump-outputs writes the native path's outputs; it does not apply to --impl reference")
     global IMAGE, CONTEXT_VIEWS
     IMAGE, CONTEXT_VIEWS = (args.image, args.image), args.context_views
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
-    if args.impl == "reference":
-        if args.steps == 400 and args.warmup == 10:
-            args.steps, args.warmup = 2, 1
+    if reference:
         run_reference(args, rank, world)
         return
     if args.warmup < 3:
@@ -359,6 +393,13 @@ def main():
         pool_dev.append(d)
     g = torch.Generator(device="cpu").manual_seed(7)
     d_img = torch.randn((1, V, 3, *IMAGE), generator=g).to(dev)
+    rows = None
+    if args.dump_outputs:               # checked on every rank: all ranks have the same shapes, so all stop together
+        rows = dump_rows(P)
+        dump_bytes = 4 * (d_img.numel() + len(rows) * sum(pool_dev[0][k][0, 0].numel() for k in GAUSS_KEYS))
+        if dump_bytes > DUMP_LIMIT:
+            raise SystemExit(f"--dump-outputs: {dump_bytes / 1e6:.0f} MB of outputs at this size, over "
+                             f"{DUMP_LIMIT / 1e6:.0f} MB (the image is written whole)")
 
     def barrier():
         if world > 1:
@@ -386,22 +427,26 @@ def main():
     launches0 = _lib.lib.ps_launch_count()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     def run_steps(n):
+        """Runs n steps; returns the (image, gradients) of the last."""
         if graphs is not None:
             for i in range(n):
                 graphs[i % args.pool][0].replay()
-        else:
-            for i in range(n):
-                render_step(pool_dev[i % args.pool], d_img, V)
+            return graphs[(n - 1) % args.pool][1]
+        for i in range(n):
+            out = render_step(pool_dev[i % args.pool], d_img, V)
+        return out
 
     with ClockSampler(local_rank) as clk:
         barrier()
         t_begin = time.monotonic()
         e0.record()
-        run_steps(K)
+        last = run_steps(K)
         e1.record()
         barrier()
         t_end = time.monotonic()
         launches_timed = _lib.lib.ps_launch_count() - launches0
+        # read now: the steps below replay the same graphs and overwrite their outputs
+        outputs = step_outputs(*last, rows) if (rows is not None and rank == 0) else None
         clock_window = "timed region"
         if clk.proc is not None and clk.count_between(t_begin, t_end) < 3:
             # the timed region is shorter than a few nvidia-smi sampling periods: keep the SAME load running,
@@ -582,6 +627,12 @@ def main():
         cpu = {"value": 1.0 / dt, "unit": UNIT, "cores": threads, "kind": "port",
                "sample": "1 view of configs[1] (256x256, P=393216) forward+backward, pure-PyTorch CPU "
                          f"oracle (oracle/raster_torch.py), torch.set_num_threads({threads}), {dt:.1f} s"}
+
+    if outputs is not None:
+        out_dir = Path(args.dump_outputs)
+        out_dir.mkdir(parents=True, exist_ok=True)
+        for name, a in outputs.items():
+            np.save(out_dir / f"{name}.npy", a)
 
     if rank == 0:
         line = {

@@ -138,9 +138,11 @@ def take(prefix: str, out: dict) -> None:
 def main():
     cs = load_reference_cuda_splatting()
     s = scene()
-    out = {}
+    # the scene goes to render_cuda_scene.npz, the recorded calls to render_cuda_args.npz (each file under 1 MB)
+    scene_out = {}
     for k, v in s.items():
-        store(out, f"scene_{k}", v[:1] if k in ("means", "covariances", "harmonics", "opacities") else v)
+        store(scene_out, f"scene_{k}", v[:1] if k in ("means", "covariances", "harmonics", "opacities") else v)
+    out = {}
     args = (s["extrinsics"], s["intrinsics"], s["near"], s["far"], s["image_shape"])
     g = (s["means"], s["covariances"], s["harmonics"], s["opacities"])
     img = cs.render_cuda(*args, s["background"], *g)
@@ -176,6 +178,7 @@ def main():
     out["proj_fov"] = fov.numpy()
     out["proj_matrix"] = cs.get_projection_matrix(s["near"], s["far"], fov[:, 0], fov[:, 1]).numpy()
     OUT.mkdir(parents=True, exist_ok=True)
+    np.savez_compressed(OUT / "render_cuda_scene.npz", **scene_out)
     np.savez_compressed(OUT / "render_cuda_args.npz", **out)
     print("wrote", OUT / "render_cuda_args.npz", len(out), "arrays;",
           {k: out[k].shape for k in ("render_cuda_0_shs", "render_cuda_0_cov3D_precomp", "render_cuda_0_viewmatrix")},

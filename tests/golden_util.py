@@ -10,15 +10,16 @@ import zlib
 import torch
 
 
-def load_npz_refs(path) -> dict:
-    """np.load of a fixture whose writer stored byte-identical large arrays once (`key__ref` names the
-    first copy; oracle/make_render_args_golden.py)."""
+def load_npz_refs(*paths) -> dict:
+    """np.load of the fixtures of one recording, merged, whose writer stored byte-identical large arrays once
+    (`key__ref` names the first copy; oracle/make_render_args_golden.py)."""
     import numpy as np
-    raw = np.load(path)
-    out = {k: raw[k] for k in raw.files if not k.endswith("__ref")}
-    for k in raw.files:
-        if k.endswith("__ref"):
-            out[k[:-5]] = out[str(raw[k])]
+    raws = [np.load(p) for p in paths]
+    out = {k: raw[k] for raw in raws for k in raw.files if not k.endswith("__ref")}
+    for raw in raws:
+        for k in raw.files:
+            if k.endswith("__ref"):
+                out[k[:-5]] = out[str(raw[k])]
     return out
 
 

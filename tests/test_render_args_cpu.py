@@ -15,7 +15,8 @@ import torch
 from oracle import raster_torch as rt
 from tests import golden_util as gu
 
-G = gu.load_npz_refs(Path(__file__).resolve().parent / "golden" / "render_cuda_args.npz")
+GOLD = Path(__file__).resolve().parent / "golden"
+G = gu.load_npz_refs(GOLD / "render_cuda_args.npz", GOLD / "render_cuda_scene.npz")
 T = lambda k: torch.from_numpy(np.asarray(G[k]))
 
 

@@ -23,7 +23,8 @@ from tests import util
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
-G = gu.load_npz_refs(Path(__file__).resolve().parent / "golden" / "render_cuda_args.npz")
+GOLD = Path(__file__).resolve().parent / "golden"
+G = gu.load_npz_refs(GOLD / "render_cuda_args.npz", GOLD / "render_cuda_scene.npz")
 H, W = 24, 40
 
 
