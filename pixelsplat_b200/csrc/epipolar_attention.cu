@@ -632,7 +632,7 @@ extern "C" PS_API int ps_epipolar_attention_backward(const ps_epipolar_desc *d, 
     int rc = epi_check(d);
     if (rc) return rc;
     if (!in || !in->features || !in->segments || !in->valid || !in->rel_disparity || !in->q_feat || !lse ||
-        !dz || (d->pe_dim > 0 && (!de || !dq_pe)) || !d_row || !dq_feat || !dfeatures) {
+        !dz || (d->pe_dim > 0 && (!in->q_pe || !de || !dq_pe)) || !d_row || !dq_feat || !dfeatures) {
         set_error("ps_epipolar_attention_backward: a required pointer is NULL");
         return PS_ERR_INVALID_ARGUMENT;
     }

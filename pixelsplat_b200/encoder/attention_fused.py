@@ -103,9 +103,23 @@ class EpipolarKV:
         return kv.permute(0, 1, 3, 4, 2, 5).reshape(b * v * r, s * ov, c)   # "(b v r) (s ov) c"
 
 
+def supported(heads: int, channels: int, samples: int, pe_dim: int, views: int) -> bool:
+    """Whether the fused kernel takes this shape: the checks of `epi_check` (csrc/epipolar_attention.cu)."""
+    return (1 <= heads <= 4 and channels == 128 and 1 <= samples <= 32 and 0 <= pe_dim <= 32
+            and pe_dim % 2 == 0 and heads * pe_dim <= 96 and 2 <= views <= 33)
+
+
+def fused_supported(attn, kv: EpipolarKV) -> bool:
+    """`supported` for the `Attention` module `attn` attending to `kv`."""
+    pe_dim = 0 if kv.depth_linear is None else kv.depth_linear.in_features
+    return supported(attn.heads, kv.features.shape[2], kv.geometry.samples, pe_dim, kv.features.shape[1])
+
+
 class _EpipolarAttentionFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, qt, pq, bias, feat_cl, geometry: EpipolarGeometry, heads: int):
+        if not feat_cl.is_cuda:
+            raise ValueError("pixelsplat_b200 has no CPU path: the epipolar attention needs CUDA tensors")
         b, v, h, w, c = feat_cl.shape
         n = b * v * h * w
         dev = feat_cl.device
@@ -136,7 +150,7 @@ class _EpipolarAttentionFn(torch.autograd.Function):
         g, desc = ctx.geometry, ctx.desc
         dev = feat_cl.device
         dz, de = dz.contiguous().float(), de.contiguous().float()
-        use_mass = ctx.has_bias and dmass is not None
+        use_mass = dmass is not None          # mass is an output with or without a bias input
         d_row = (dz * z).sum(-1) + (de * e).sum(-1)
         if use_mass:
             dmass = dmass.contiguous().float()
@@ -158,9 +172,8 @@ class _EpipolarAttentionFn(torch.autograd.Function):
 
 
 def fused_epipolar_attention(attn, x: Tensor, kv: EpipolarKV) -> Tensor:
-    """attn: the `Attention` module (to_q / to_kv / to_out); x: [n, 1, c] (already layer-normed)."""
-    if not x.is_cuda:
-        raise ValueError("pixelsplat_b200 has no CPU path: the epipolar attention needs CUDA tensors")
+    """attn: the `Attention` module (to_q / to_kv / to_out); x: [n, 1, c] (already layer-normed).
+    The shape must pass `fused_supported(attn, kv)`."""
     n, one, c = x.shape
     assert one == 1
     H, d = attn.heads, attn.dim_head

@@ -7,7 +7,9 @@ are then never materialised -- the fused CUDA kernel gathers them from the featu
 (pixelsplat_b200/encoder/attention_fused.py).  If a forward hook is registered on `attend` (the
 reference's visualisers hook `transformer.layers[i][0].fn.attend`,
 encoder_visualizer_epipolar.py:53-56) the module falls back to the explicit soft-max path so the
-hook sees the [(b v r), head, 1, s*ov] attention tensor it expects.
+hook sees the [(b v r), head, 1, s*ov] attention tensor it expects.  It takes the same explicit path for
+shapes the kernel does not cover (more than 4 heads or 32 samples, features other than 128 channels,
+a depth encoding wider than the kernel's; `attention_fused.supported`), which the reference accepts.
 
 With z = None (ImageSelfAttention's ViT blocks) and the shape the kernel is written for (256 tokens,
 128-dim heads) the soft-max attention runs on the tcgen05 tensor cores
@@ -19,7 +21,7 @@ import torch
 from torch import Tensor, nn
 
 from . import self_attention_tc as _satc
-from .attention_fused import EpipolarKV, fused_epipolar_attention
+from .attention_fused import EpipolarKV, fused_epipolar_attention, fused_supported
 
 
 class Attention(nn.Module):
@@ -46,7 +48,7 @@ class Attention(nn.Module):
     def forward(self, x: Tensor, z=None) -> Tensor:
         if isinstance(z, EpipolarKV):
             hooked = len(self.attend._forward_hooks) > 0 or len(self.attend._forward_pre_hooks) > 0
-            if not hooked and isinstance(self.to_out, nn.Sequential):
+            if not hooked and isinstance(self.to_out, nn.Sequential) and fused_supported(self, z):
                 return fused_epipolar_attention(self, x, z)
             z = z.materialize()
         if z is None:
